@@ -52,7 +52,22 @@ def parse():
     ap.add_argument("--cpu-n", type=int, default=16000, help="cloud size of the bounded CPU sample")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-e2e", action="store_true")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the potentials of the last timed step to DIR/<name>.npy (float32)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
+
+
+def dump_outputs(out_dir, pots):
+    """The four potentials (f_ba, g_ab, f_aa, g_bb) the last timed step returned: 4 (N,) float32 arrays, 16 MB at the
+    default N = 1e6.  The inputs are seeded, so two builds run with the same arguments can be compared array by array."""
+    import numpy as np
+
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in pots.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.detach().float().cpu().numpy().reshape(-1))
 
 
 # ----------------------------------------------------------------------------------------------------
@@ -210,6 +225,8 @@ def run_reference(args):
         for _ in range(args.steps):
             pots = dense_iteration(O, eps, a_log, C, pots)
         dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, pots)
     pairs = 4.0 * n * n
     value = pairs * args.steps / dt
     cores = torch.get_num_threads()
@@ -312,6 +329,8 @@ def run_b200(args):
             ev[k][1].record()
         sync_all()
     step_ms = [a.elapsed_time(b) for a, b in ev]
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, pots)
     total_ms = torch.tensor([sum(step_ms)], device=dev, dtype=torch.float64)
     if world > 1:
         dist.all_reduce(total_ms, op=dist.ReduceOp.MAX)

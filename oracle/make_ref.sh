@@ -7,9 +7,7 @@
 # Nothing is copied into the tracked tree: pip builds a wheel from a scratch copy under /tmp (the reference mount is
 # read-only) and unpacks it under oracle/_ref/.  Used by
 #   * bench.py --impl reference  ->  cpu_baseline.kind = "reference": the reference's own softmin_tensorized /
-#     cost routines timed on the host cores;
-#   * tests/test_live_reference.py: the CUDA engine against the LIVE reference (tensorized on CPU, and its pykeops
-#     backends on tests/golden/pykeops_shim) on fresh random inputs.
+#     cost routines timed on the host cores.
 set -euo pipefail
 HERE="$(cd "$(dirname "$0")" && pwd)"
 SRC="${GEOMLOSS_REFERENCE_ROOT:-/root/reference}"
