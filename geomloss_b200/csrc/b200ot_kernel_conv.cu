@@ -67,18 +67,22 @@ __global__ void conv_fwd_finalize_kernel(const float* __restrict__ part, int n_s
 
 // gaussian: part (n_split, N, D+1): [0] = sum W e, [1+k] = sum W e Y_k   -> go (accY - X acc0) / (scale blur^2)
 // laplacian / energy: part (n_split, N, D): sum W e u_k                    -> -go acc / blur   (energy: -go acc)
+// laplacian / energy on the tensor cores (coord_absmax != null): part (n_split, N, D+1) as for the gaussian, with
+//   X = (x - c) / s and P = w k'(r)/r up to the factor -coef (tcbwd.cuh, MODE 4 / 5)     -> go coef (accY - X acc0)
 __global__ void conv_bwd_finalize_kernel(const float* __restrict__ part, int n_split, const float* __restrict__ x,
                                          const float* __restrict__ center, const float* __restrict__ grad_out,
                                          float* __restrict__ grad_x, int64_t N, int D, int kind, float scale,
                                          float coef, const float* __restrict__ w_absmax,
-                                         float* __restrict__ value_out = nullptr) {
+                                         float* __restrict__ value_out = nullptr,
+                                         const float* __restrict__ coord_absmax = nullptr) {
   const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= N) return;
+  if (coord_absmax != nullptr) scale = tc_coord_inv(coord_absmax);
   float go = grad_out ? grad_out[i] : 1.f;  // no upstream gradient: the unit row gradient (value + gradient pass)
   float wmax = 1.f;
   if (w_absmax != nullptr && *w_absmax > 0.f) wmax = *w_absmax;  // tensor-core path: weights were normalised
   go *= wmax;
-  if (kind == B200OT_KERNEL_GAUSSIAN) {
+  if (kind == B200OT_KERNEL_GAUSSIAN || coord_absmax != nullptr) {
     const int na = D + 1;
     float a0 = 0.f;
     for (int s = 0; s < n_split; ++s) a0 += part[((int64_t)s * N + i) * na];
@@ -107,6 +111,21 @@ __global__ void absmax_kernel(const float* __restrict__ w, int64_t n, float* __r
 #pragma unroll
   for (int o = 16; o > 0; o >>= 1) m = fmaxf(m, __shfl_xor_sync(0xffffffffu, m, o));
   if ((threadIdx.x & 31) == 0 && m > 0.f && !(m != m)) atomicMax(reinterpret_cast<unsigned int*>(out), __float_as_uint(m));
+}
+
+// max_k |x_ik - c_k| over the rows of x:(n, D) and y:(m, D) into *out (zero-initialised by the caller): the coordinate
+// scale s of the tensor-core laplacian / energy kernels (tcconv.cuh: tc_coord_scale)
+__global__ void coord_absmax_kernel(const float* __restrict__ x, int64_t n, const float* __restrict__ y, int64_t m,
+                                    int D, const float* __restrict__ center, float* __restrict__ out) {
+  float v = 0.f;
+  const int64_t nx = n * D, total = nx + m * D;
+  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (int64_t)gridDim.x * blockDim.x) {
+    const float p = i < nx ? x[i] : y[i - nx];
+    v = fmaxf(v, fabsf(p - (center ? center[i % D] : 0.f)));
+  }
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) v = fmaxf(v, __shfl_xor_sync(0xffffffffu, v, o));
+  if ((threadIdx.x & 31) == 0 && v > 0.f) atomicMax(reinterpret_cast<unsigned int*>(out), __float_as_uint(v));
 }
 
 template <int MODE, int D>
@@ -176,7 +195,7 @@ static float conv_bwd_coef(int kind_flags, const ConvScales& cs, float blur) {
 }
 
 // ---------------------------------------------------------------------------------------------------
-// tensor-core path (gaussian, 8 < D <= 64): see tcconv.cuh
+// tensor-core path (gaussian; laplacian / energy above B200OT_MAX_D), 8 < D <= 64: see tcconv.cuh
 // ---------------------------------------------------------------------------------------------------
 constexpr int kTcBN = 128;    // columns per MMA tile
 constexpr int kTcEpi = 16;    // epilogue warps of the forward kernels: 4 per TMEM lane quarter hide the tcgen05.ld latency
@@ -293,17 +312,52 @@ int64_t tc_scratch_bytes(int64_t N, int64_t M, int D) {
   return std::max(make_tc_plan(N, M, D, false).total, make_tc_plan(N, M, D, true).total);
 }
 
-// Row gradients on the tensor-core path (gaussian conv: kind 0 / softmin p=2: kind 1).  Leaves n_part sets of
-// (N, D+1) partial sums in *part_out.
+// Laplacian / energy on the tensor cores (tcconv.cuh / tcbwd.cuh, MODE 4 / 5): the exponent factor per unit of
+// distance and the clamp on |x - y|^2 in the units of x.  The pykeops convention (UNCLAMPED) clamps at exactly 0:
+// r = 0 and a zero gradient at coincident points.
+struct TcSqrtParams {
+  float kc, clampq;
+};
+static TcSqrtParams tc_sqrt_params(int kind_flags, float blur) {
+  const float clamp = (kind_flags & B200OT_KERNEL_UNCLAMPED) ? 0.f : cost_clamp(kind_flags);
+  if (kind_base(kind_flags) == B200OT_KERNEL_LAPLACIAN) return {kLog2e / blur, clamp * blur * blur};
+  return {0.f, clamp};
+}
+
+// The coordinate scale s of the sqrt kernels, max |x - c| over both clouds, into the plan's misc block (behind
+// max|w|): energy has no exponent to bound |X| (the gaussian pack's +-60000 clamp would cut real coordinates), and
+// with |X| <= 1 every fp16 operand term is in range whatever the units of the data.
+static int tc_coord_absmax(const TcPlan& p, unsigned char* base, const float* x, int64_t N, const float* y, int64_t M,
+                           int D, const float* center, cudaStream_t st, const float** out) {
+  float* s = reinterpret_cast<float*>(base + p.off_misc) + 1;
+  B200OT_CUDA_TRY(cudaMemsetAsync(s, 0, sizeof(float), st));
+  coord_absmax_kernel<<<(unsigned)std::min<int64_t>(ceil_div64((N + M) * D, 256), 1024), 256, 0, st>>>(x, N, y, M, D,
+                                                                                                      center, s);
+  B200OT_CUDA_TRY(cudaGetLastError());
+  *out = s;
+  return B200OT_OK;
+}
+
+// Row gradients on the tensor-core path (kind 0: gaussian conv, 1: softmin p=2, 2 / 3: laplacian / energy conv with
+// tc_sqrt_params (kc, clampq); their coordinate scale is returned in *coord_out for the finalize).  Leaves n_part sets
+// of (N, D+1) partial sums in *part_out.
 int bwd_partial_tc(int kind, const float* x, const float* y, const float* w, const float* h_a, const float* h_b,
                    float h_scale_b, const float* lse2, const float* center, float scale, int64_t N, int64_t M, int D,
-                   void* scratch, float** part_out, int* n_part_out, cudaStream_t st, const float** w_absmax_out) {
+                   void* scratch, float** part_out, int* n_part_out, cudaStream_t st, const float** w_absmax_out,
+                   float kc, float clampq, const float** coord_out) {
   const TcPlan p = make_tc_plan(N, M, D, true);
   if (p.nstage < 1) return B200OT_EINVAL;
   unsigned char* base = reinterpret_cast<unsigned char*>(scratch);
   unsigned char* a_imgs = base;
   unsigned char* b_imgs = base + p.off_b;
   float* part = reinterpret_cast<float*>(base + p.off_part);
+  const bool sqrt_kind = kind >= 2;
+  const float* coord = nullptr;
+  if (sqrt_kind) {
+    const int rc = tc_coord_absmax(p, base, x, N, y, M, D, center, st, &coord);
+    if (rc) return rc;
+  }
+  if (coord_out) *coord_out = coord;
   float* w_absmax = nullptr;
   if (w != nullptr) {
     // P = w_j e_ij feeds an fp16 GEMM: normalise the weights to max|w| = 1 (undone by the finalize kernel)
@@ -315,18 +369,20 @@ int bwd_partial_tc(int kind, const float* x, const float* y, const float* w, con
   if (w_absmax_out) *w_absmax_out = w_absmax;
   const int threads = 128;
   tc_pack_kernel<<<(unsigned)ceil_div64(p.a_tiles_pad * kTcM, threads), threads, 0, st>>>(
-      x, nullptr, nullptr, nullptr, 0.f, 0.f, center, scale, N, D, p.kp, kTcM, 0, a_imgs, lse2, nullptr, kTcRT);
+      x, nullptr, nullptr, nullptr, 0.f, 0.f, center, scale, N, D, p.kp, kTcM, 0, a_imgs, lse2, nullptr, kTcRT,
+      coord);
   B200OT_CUDA_TRY(cudaGetLastError());
   tc_pack_kernel<<<(unsigned)ceil_div64(p.b_tiles * kTcBN, threads), threads, 0, st>>>(
-      y, w, h_a, h_b, h_scale_b, kLog2e, center, scale, M, D, p.kp, kTcBN, 1, b_imgs, nullptr, w_absmax);
+      y, w, h_a, h_b, h_scale_b, kLog2e, center, scale, M, D, p.kp, kTcBN, 1, b_imgs, nullptr, w_absmax, 1, coord);
   B200OT_CUDA_TRY(cudaGetLastError());
   dim3 grid((unsigned)p.a_tiles, (unsigned)p.n_split);
-  const int self_mode = (kind == 0 && x == y && N == M) ? 1 : 0;  // K_xx: exact zero exponent on the diagonal
+  // K_xx: exact zero exponent (gaussian) / zero gradient (laplacian, energy) on the diagonal
+  const int self_mode = (kind != 1 && x == y && N == M) ? 1 : 0;
   const TcBwdTuning tn = tc_bwd_tuning();
   auto launch = [&](auto kern, int threads) -> int {
     B200OT_CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)p.smem));
     kern<<<grid, threads, (size_t)p.smem, st>>>(a_imgs, b_imgs, part, N, p.kp, (int)p.b_tiles, p.tiles_per_split,
-                                                p.nstage, D, self_mode);
+                                                p.nstage, D, self_mode, kc, clampq, coord);
     B200OT_CUDA_TRY(cudaGetLastError());
     return B200OT_OK;
   };
@@ -345,7 +401,13 @@ int bwd_partial_tc(int kind, const float* x, const float* y, const float* w, con
       return tn.p_terms == 1 ? pick3(mode_tag, T1{}, std::true_type{}) : pick3(mode_tag, T2{}, std::true_type{});
     return tn.p_terms == 1 ? pick3(mode_tag, T1{}, std::false_type{}) : pick3(mode_tag, T2{}, std::false_type{});
   };
-  const int rc = (kind == 0) ? pick(std::integral_constant<int, 2>{}) : pick(std::integral_constant<int, 3>{});
+  int rc;
+  switch (kind) {
+    case 0: rc = pick(std::integral_constant<int, 2>{}); break;
+    case 1: rc = pick(std::integral_constant<int, 3>{}); break;
+    case 2: rc = pick(std::integral_constant<int, 4>{}); break;
+    default: rc = pick(std::integral_constant<int, 5>{}); break;
+  }
   if (rc) return rc;
   *part_out = part;
   *n_part_out = p.n_split;  // G of a CTA is complete over its column split (both column halves feed one GEMM)
@@ -375,15 +437,17 @@ int softmin_partial_tc(const float* x, const float* y, const float* h_a, const f
   B200OT_CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)p.smem));
   dim3 grid((unsigned)(p.a_tiles_pad / kTcRT), (unsigned)p.n_split);
   kern<<<grid, TcConvCfg::THREADS, (size_t)p.smem, st>>>(a_imgs, b_imgs, part, N, p.kp, (int)p.b_tiles,
-                                                        p.tiles_per_split, p.nstage, D, 0);
+                                                        p.tiles_per_split, p.nstage, D, 0, 0.f, 0.f, nullptr);
   B200OT_CUDA_TRY(cudaGetLastError());
   *part_out = part;
   *n_part_out = p.n_split * (kTcEpi / 4);
   return B200OT_OK;
 }
 
-static int conv_fwd_tc(const float* x, const float* y, const float* w, const float* center, float* out, int64_t N,
-                       int64_t M, int D, float blur, void* scratch, cudaStream_t st) {
+// kind_flags: gaussian (MODE 0), laplacian (MODE 4) or energy (MODE 5), with or without B200OT_KERNEL_UNCLAMPED
+static int conv_fwd_tc(int kind_flags, const float* x, const float* y, const float* w, const float* center, float* out,
+                       int64_t N, int64_t M, int D, float blur, void* scratch, cudaStream_t st) {
+  const int kind = kind_base(kind_flags);
   const int self_mode = (x == y && N == M) ? 1 : 0;  // K_xx / K_yy: the diagonal exponent is exactly 0 (tcconv.cuh)
   const TcPlan p = make_tc_plan(N, M, D);
   if (p.nstage < 1) return B200OT_EINVAL;
@@ -391,22 +455,32 @@ static int conv_fwd_tc(const float* x, const float* y, const float* w, const flo
   unsigned char* a_imgs = base;
   unsigned char* b_imgs = base + p.off_b;
   float* part = reinterpret_cast<float*>(base + p.off_part);
-  const float scale = sqrtf(kLog2e) / blur;
+  const bool gauss = kind == B200OT_KERNEL_GAUSSIAN;
+  const float scale = gauss ? sqrtf(kLog2e) / blur : 1.f;
+  const TcSqrtParams sq = gauss ? TcSqrtParams{0.f, 0.f} : tc_sqrt_params(kind_flags, blur);
+  const float* coord = nullptr;
+  if (!gauss) {
+    const int rc = tc_coord_absmax(p, base, x, N, y, M, D, center, st, &coord);
+    if (rc) return rc;
+  }
   const int threads = 128;
   tc_pack_kernel<<<(unsigned)ceil_div64(p.a_tiles_pad * kTcM, threads), threads, 0, st>>>(
-      x, nullptr, nullptr, nullptr, 0.f, 0.f, center, scale, N, D, p.kp, kTcM, 0, a_imgs, nullptr, nullptr, kTcRT);
+      x, nullptr, nullptr, nullptr, 0.f, 0.f, center, scale, N, D, p.kp, kTcM, 0, a_imgs, nullptr, nullptr, kTcRT,
+      coord);
   B200OT_CUDA_TRY(cudaGetLastError());
   tc_pack_kernel<<<(unsigned)ceil_div64(p.b_tiles * kTcBN, threads), threads, 0, st>>>(
-      y, w, nullptr, nullptr, 0.f, 0.f, center, scale, M, D, p.kp, kTcBN, 1, b_imgs);
+      y, w, nullptr, nullptr, 0.f, 0.f, center, scale, M, D, p.kp, kTcBN, 1, b_imgs, nullptr, nullptr, 1, coord);
   B200OT_CUDA_TRY(cudaGetLastError());
-  auto kern = tc_reduce_kernel<TcConvCfg, 0>;
+  auto kern = gauss ? tc_reduce_kernel<TcConvCfg, 0>
+                    : (kind == B200OT_KERNEL_LAPLACIAN ? tc_reduce_kernel<TcConvCfg, 4> : tc_reduce_kernel<TcConvCfg, 5>);
   B200OT_CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)p.smem));
   dim3 grid((unsigned)(p.a_tiles_pad / kTcRT), (unsigned)p.n_split);
   kern<<<grid, TcConvCfg::THREADS, (size_t)p.smem, st>>>(a_imgs, b_imgs, part, N, p.kp, (int)p.b_tiles,
-                                                        p.tiles_per_split, p.nstage, D, self_mode);
+                                                        p.tiles_per_split, p.nstage, D, self_mode, sq.kc, sq.clampq,
+                                                        coord);
   B200OT_CUDA_TRY(cudaGetLastError());
-  conv_fwd_finalize_kernel<<<(unsigned)ceil_div64(N, 256), 256, 0, st>>>(part, p.n_split * (kTcEpi / 4), 1.f, out,
-                                                                       N);
+  conv_fwd_finalize_kernel<<<(unsigned)ceil_div64(N, 256), 256, 0, st>>>(
+      part, p.n_split * (kTcEpi / 4), kind == B200OT_KERNEL_ENERGY ? -1.f : 1.f, out, N);
   B200OT_CUDA_TRY(cudaGetLastError());
   return B200OT_OK;
 }
@@ -481,16 +555,23 @@ B200OT_API int b200ot_kernel_conv_partial_ranges(const float* x, const float* ce
                       reinterpret_cast<const int2*>(pieces));
 }
 
+// Laplacian / energy take the tensor cores above B200OT_MAX_D only: at D <= B200OT_MAX_D they stay on the CUDA cores
+// whatever $B200OT_TC_MIN_D / $B200OT_TC_MIN_PAIRS say (tc_routed's cross-over was measured for the gaussian).
+static bool conv_tc(int op, int kind_flags, int D, int64_t N, int64_t M) {
+  if (kind_base(kind_flags) == B200OT_KERNEL_GAUSSIAN) return tc_routed(op, D, N, M);
+  return D > B200OT_MAX_D && tc_capable_dim(D);
+}
+
 B200OT_API int b200ot_kernel_conv_fwd(const float* x, const float* y, const float* w, const float* center,
                                       float* out, int64_t N, int64_t M, int32_t D, int32_t kind, float blur,
                                       void* scratch, int64_t scratch_bytes, void* stream) {
-  const bool tc = (kind_base(kind) == B200OT_KERNEL_GAUSSIAN) && tc_routed(kTcConvFwd, D, N, M);
+  const bool tc = conv_tc(kTcConvFwd, kind, D, N, M);
   if (!x || !y || !w || !out || !scratch || N <= 0 || M <= 0 || (!supported_simt_dim(D) && !tc) || !valid_kind(kind))
     return B200OT_EINVAL;
   if (kind_base(kind) != B200OT_KERNEL_ENERGY && !(blur > 0.f)) return B200OT_EINVAL;
   if (((uintptr_t)scratch) & 15) return B200OT_EALIGN;
   if (scratch_bytes < b200ot_kernel_conv_scratch_bytes(N, M, D)) return B200OT_ESCRATCH;
-  if (tc) return conv_fwd_tc(x, y, w, center, out, N, M, D, blur, scratch, (cudaStream_t)stream);
+  if (tc) return conv_fwd_tc(kind, x, y, w, center, out, N, M, D, blur, scratch, (cudaStream_t)stream);
   const ReducePlan pl = make_plan(N, M, D);
   const ConvScales cs = conv_scales(kind, blur);
   float* cols = reinterpret_cast<float*>(scratch);
@@ -509,13 +590,30 @@ static int conv_bwd_x_impl(const float* x, const float* y, const float* w, const
                            float* grad_x, float* value_out, int64_t N, int64_t M, int32_t D, int32_t kind, float blur,
                            void* scratch, int64_t scratch_bytes, void* stream) {
   const bool gauss = kind_base(kind) == B200OT_KERNEL_GAUSSIAN;
-  const bool tc = gauss && tc_routed(kTcConvBwd, D, N, M);
+  const bool tc = conv_tc(kTcConvBwd, kind, D, N, M);
   if (!x || !y || !w || !grad_x || !scratch || N <= 0 || M <= 0 || (!supported_simt_dim(D) && !tc) ||
       !valid_kind(kind) || (value_out && !gauss))
     return B200OT_EINVAL;
   if (kind_base(kind) != B200OT_KERNEL_ENERGY && !(blur > 0.f)) return B200OT_EINVAL;
   if (((uintptr_t)scratch) & 15) return B200OT_EALIGN;
   if (scratch_bytes < b200ot_kernel_conv_scratch_bytes(N, M, D)) return B200OT_ESCRATCH;
+  if (tc && !gauss) {
+    // P = w k'(r)/r without its negative factor (tcbwd.cuh): grad = go (-k'(r)/r factor) (sum P Y - X sum P)
+    float* tc_part = nullptr;
+    int n_part = 0;
+    const float* w_absmax = nullptr;
+    const float* coord = nullptr;
+    const TcSqrtParams sq = tc_sqrt_params(kind, blur);
+    const bool lap = kind_base(kind) == B200OT_KERNEL_LAPLACIAN;
+    const int rc = bwd_partial_tc(lap ? 2 : 3, x, y, w, nullptr, nullptr, 0.f, nullptr, center, 1.f, N, M, D, scratch,
+                                  &tc_part, &n_part, (cudaStream_t)stream, &w_absmax, sq.kc, sq.clampq, &coord);
+    if (rc) return rc;
+    conv_bwd_finalize_kernel<<<(unsigned)ceil_div64(N, 256), 256, 0, (cudaStream_t)stream>>>(
+        tc_part, n_part, x, center, grad_out, grad_x, N, D, kind_base(kind), 1.f, lap ? 1.0f / blur : 1.0f, w_absmax,
+        nullptr, coord);
+    B200OT_CUDA_TRY(cudaGetLastError());
+    return B200OT_OK;
+  }
   if (tc) {
     float* tc_part = nullptr;
     int n_part = 0;

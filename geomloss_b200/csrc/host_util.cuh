@@ -54,7 +54,8 @@ int softmin_partial_tc(const float* x, const float* y, const float* h_a, const f
 
 int bwd_partial_tc(int kind, const float* x, const float* y, const float* w, const float* h_a, const float* h_b,
                    float h_scale_b, const float* lse2, const float* center, float scale, int64_t N, int64_t M, int D,
-                   void* scratch, float** part_out, int* n_part_out, cudaStream_t st, const float** w_absmax_out);
+                   void* scratch, float** part_out, int* n_part_out, cudaStream_t st, const float** w_absmax_out,
+                   float kc = 0.f, float clampq = 0.f, const float** coord_out = nullptr);
 
 #define B200OT_STR2(x) #x
 #define B200OT_STR(x) B200OT_STR2(x)

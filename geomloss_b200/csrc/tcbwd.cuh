@@ -67,14 +67,29 @@ __host__ __device__ constexpr uint32_t make_idesc_f16_bmn(int M, int N) { return
 // LDALL (8 epilogue warps: a warp owns 64 columns of a tile): the two 32-column chunks come from one
 // tcgen05.ld.x64 instead of two x32 round trips.
 //
+// MODE 4 / 5: laplacian / energy row gradient.  d/dx_i sum_j w_j k(r_ij) = sum_j w_j k'(r_ij)/r_ij (x_i - y_j), so
+// P_ij = w_j k'(r)/r makes the same (N, D+1) sums as MODE 2.  With X = (x - c)/s (|X| <= 1, tc_pack_kernel's
+// coord_absmax) and r in units of s, the kernel feeds GEMM 2 with
+//   P_ij = w_j min(1/r_ij, 1/rho) (* 2^(-kc s r_ij), laplacian)      rho = kTcSqrtRho
+// and the negative factor -1 (energy) or -1/blur (laplacian) goes into the finalize's coefficient; the 1/s of 1/r
+// and the s of (x_i - y_j) cancel.  P <= 1/rho = 2^14 (fp16 range) and the typical pair (r ~ 1) is in fp16's normal
+// range.  Pairs with r < rho (2^-14 of the extent of the clouds: far below the ~1e-3 to which the fp32 expansion
+// resolves r near 0) count with weight 1/rho instead of 1/r.  Pairs inside the clamp (-2 S <= clampq / s^2: the
+// reference's clamp_min, pykeops' zero gradient at r = 0) contribute exactly zero.
+//
 // self_mode: rows and columns are the same cloud (the K_xx term): the exponent of pair (i, i) is exactly 0, as in
 // tc_reduce_kernel — matters when sum_j P_ij is used as the forward VALUE (b200ot_kernel_conv_fwd_bwd_x).
+constexpr float kTcSqrtRho = 1.0f / 16384.0f;
+
 template <class C, int MODE, int PT, bool LDALL, bool MERGE>
 __global__ void __launch_bounds__(C::THREADS, 1)
     tc_bwd_kernel(const unsigned char* __restrict__ a_imgs, const unsigned char* __restrict__ b_imgs,
                   float* __restrict__ part, int64_t N, int kp, int ntiles_b, int tiles_per_split, int NSTAGE, int D,
-                  int self_mode) {
+                  int self_mode, float kc = 0.f, float clampq = 0.f,
+                  const float* __restrict__ coord_absmax = nullptr) {
   static_assert(PT == 1 || PT == 2, "P is fed to GEMM 2 as one or two fp16 terms");
+  static_assert(MODE >= 2 && MODE <= 5, "forward reductions live in tcconv.cuh");
+  constexpr bool SQRT = MODE >= 4;
   constexpr int BN = C::BN, NEPI = C::NEPI, NACC = 2;
   static_assert(BN == 128 && (NEPI == 8 || NEPI == 16), "layout below assumes 128-column tiles, 8 or 16 epilogue warps");
   constexpr int NH = NEPI / 4;   // warps per TMEM lane quarter = column shares of a tile
@@ -228,6 +243,12 @@ __global__ void __launch_bounds__(C::THREADS, 1)
       __syncwarp();
       if (lane == 0) mbar_arrive(bar_a);
     }
+    float cq = 0.f, c2 = 0.f;  // sqrt kernels: clamp on the scaled d^2, exponent per unit of r
+    if constexpr (SQRT) {
+      const float cs = tc_coord_scale(coord_absmax);
+      cq = clampq / cs / cs;
+      c2 = -kc * cs;
+    }
     float sum0 = 0.f, sum1 = 0.f;
     for (int k = 0; k < nt; ++k) {
       const int st = k % NSTAGE, acc = k % NACC;
@@ -236,7 +257,7 @@ __global__ void __launch_bounds__(C::THREADS, 1)
       const float* wts = reinterpret_cast<const float*>(sb + st * b_bytes + BN * kp * 2);
       // one 32-column chunk of S -> P, in place; v = the chunk's exponents (registers)
       auto chunk = [&](float* v, const int col0) {
-        if constexpr (MODE == 2) {
+        if constexpr (MODE != 3) {
           if (self_mode) {
             // warp-uniform: does this 32-column chunk meet the diagonal of this warp's 32 rows?
             const int64_t gcol0 = (int64_t)(t0 + k) * BN + col0;
@@ -253,8 +274,25 @@ __global__ void __launch_bounds__(C::THREADS, 1)
         float cs0 = 0.f, cs1 = 0.f;  // per-chunk sums (two-level accumulation, like the forward kernel's per-tile sums)
 #pragma unroll
         for (int c = 0; c < 32; c += 2) {
-          float p0 = ex2_approx(v[c]), p1 = ex2_approx(v[c + 1]);
-          if constexpr (MODE == 2) {
+          float p0, p1;
+          if constexpr (SQRT) {
+            const float d0 = -2.f * v[c], d1 = -2.f * v[c + 1];
+            const float q0 = rsqrt_approx(fmaxf(d0, kTcSqrtRho * kTcSqrtRho));  // min(1/r, 1/rho)
+            const float q1 = rsqrt_approx(fmaxf(d1, kTcSqrtRho * kTcSqrtRho));
+            p0 = q0;
+            p1 = q1;
+            if constexpr (MODE == 4) {
+              p0 *= ex2_approx(c2 * (d0 * q0));  // r = d^2 min(1/r, 1/rho): exact for r >= rho
+              p1 *= ex2_approx(c2 * (d1 * q1));
+            }
+            // (selected after the exponential: at d^2 < 0 (rounding) it may overflow)
+            p0 = d0 > cq ? p0 : 0.f;
+            p1 = d1 > cq ? p1 : 0.f;
+          } else {
+            p0 = ex2_approx(v[c]);
+            p1 = ex2_approx(v[c + 1]);
+          }
+          if constexpr (MODE != 3) {
             const float2 w = *reinterpret_cast<const float2*>(wts + col0 + c);
             p0 *= w.x;
             p1 *= w.y;

@@ -46,6 +46,14 @@ __host__ __device__ inline int64_t tc_a_img_bytes(int kp) { return (int64_t)kTcM
 // column image: bf16 operand data | fp32 weights
 __host__ __device__ inline int64_t tc_b_img_bytes(int kp, int bn) { return (int64_t)bn * kp * 2 + (int64_t)bn * 4; }
 
+// Laplacian / energy kernels: the coordinate scale s = max |x - c| over both clouds, computed on the device into the
+// plan's misc block.  1/s as the pack kernel and the finalize both see it (bit-identical X in the two places).
+__device__ inline float tc_coord_scale(const float* s_ptr) {
+  const float s = *s_ptr;
+  return (s > 0.f && s <= 3.0e38f) ? s : 1.f;  // all points on the centre (or a non-finite input): unit scale
+}
+__device__ inline float tc_coord_inv(const float* s_ptr) { return 1.f / tc_coord_scale(s_ptr); }
+
 // ---------------------------------------------------------------------------------------------------
 // pack: one thread per (padded) point; writes its 16-byte piece of every K chunk of its tile image
 // ---------------------------------------------------------------------------------------------------
@@ -62,14 +70,19 @@ __device__ __forceinline__ uint4 pack8_f16(const __half* src) {
 //   c_j = h_scale * (h_a[j] + h_scale_b * h_b[j]) - |Y_j|^2 / 2      (h_a null: just the fold)
 // in the rank-one chunk, and the fp32 weight w_j (kernel conv) behind the bf16 data.  Padding columns get
 // c = -1e38 when h_a is given (softmin: they must vanish from the log-sum-exp) and w = 0 otherwise.
+//
+// coord_absmax (laplacian / energy): the device-side extent s of both clouds (coord_absmax_kernel); coordinates are
+// then X = scale / s * (x - c), i.e. |X| <= scale, and the epilogues / finalize undo the 1/s.
 static __global__ void tc_pack_kernel(const float* __restrict__ pts, const float* __restrict__ w,
                                       const float* __restrict__ h_a, const float* __restrict__ h_b,
                                       float h_scale_b, float h_scale, const float* __restrict__ center,
                                       float scale, int64_t n, int D, int kp, int tile, int is_cols,
                                       unsigned char* __restrict__ out,
                                       const float* __restrict__ row_extra = nullptr,
-                                      const float* __restrict__ w_absmax = nullptr, int pad_tiles = 1) {
+                                      const float* __restrict__ w_absmax = nullptr, int pad_tiles = 1,
+                                      const float* __restrict__ coord_absmax = nullptr) {
   const int64_t p = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (coord_absmax != nullptr) scale *= tc_coord_inv(coord_absmax);
   const int64_t group = (int64_t)tile * pad_tiles;  // images are written for a multiple of pad_tiles tiles
   const int64_t npad = ((n + group - 1) / group) * group;
   if (p >= npad) return;
@@ -88,10 +101,14 @@ static __global__ void tc_pack_kernel(const float* __restrict__ pts, const float
       float X = 0.f;
       if (live && d < D) X = scale * (pts[p * D + d] - (center ? center[d] : 0.f));
       X = fminf(fmaxf(X, -60000.f), 60000.f);  // fp16 range (only reached when every exponent underflows anyway)
-      sq = fmaf(X, X, sq);
       const __half h = __float2half_rn(X);
+      const __half l = __float2half_rn(X - __half2float(h));
+      // sqrt kernels: |X|^2 of the value the MMAs multiply (h + l, 22 bits) — with the fp32 X the expansion would
+      // carry a 2^-22 |X|^2 bias in d^2, which sqrt turns into a relative error of r at near-coincident pairs
+      const float Xq = (coord_absmax != nullptr) ? __half2float(h) + __half2float(l) : X;
+      sq = fmaf(Xq, Xq, sq);
       term[0][k] = h;
-      term[1][k] = __float2half_rn(X - __half2float(h));
+      term[1][k] = l;
     }
 #pragma unroll
     for (int s = 0; s < kTcTerms; ++s)
@@ -161,7 +178,11 @@ struct TcCfg {
 // MODE 0: gaussian kernel conv  part[(split*NH + half)*N + row]   = sum_j w_j 2^S_ij
 // MODE 1: softmin               part2[(split*NH + half)*N + row]  = (m, s) with sum_j 2^S_ij = s 2^m  (lazy max,
 //         sum-guarded exactly like softmin.cuh; same partial format as softmin_partial_kernel)
-// (row gradients — modes 2 and 3 — are a two-GEMM kernel of their own: tcbwd.cuh)
+// MODE 4: laplacian kernel conv  part[...] = sum_j w_j 2^(-kc s r_ij)      r = sqrt(max(-2 S_ij, clampq / s^2))
+// MODE 5: energy kernel conv     part[...] = s sum_j w_j r_ij              (the caller negates: k = -|x - y|)
+//         S is accumulated on coordinates X = (x - c) / s (|X| <= 1: tc_pack_kernel's coord_absmax), so r is the
+//         distance in units of s; kc = log2(e) / blur; clampq = the clamp on |x - y|^2 in the units of x.
+// (row gradients — modes 2 and 3, 4 and 5 — are a two-GEMM kernel of their own: tcbwd.cuh)
 //
 // A CTA owns kTcRT = 2 row tiles (2 x 128 rows) and ping-pongs between them: step (k, r) multiplies row tile r by
 // column tile k into accumulator r, so (i) every column tile fetched from L2 feeds 2 x 128 rows — at one row tile
@@ -172,9 +193,11 @@ template <class C, int MODE>
 __global__ void __launch_bounds__(C::THREADS, 1)
     tc_reduce_kernel(const unsigned char* __restrict__ a_imgs, const unsigned char* __restrict__ b_imgs,
                      float* __restrict__ part, int64_t N, int kp, int ntiles_b, int tiles_per_split, int NSTAGE,
-                     int D, int self_mode) {
+                     int D, int self_mode, float kc = 0.f, float clampq = 0.f,
+                     const float* __restrict__ coord_absmax = nullptr) {
   constexpr int BN = C::BN, NEPI = C::NEPI, RT = kTcRT;
-  static_assert(MODE == 0 || MODE == 1, "row gradients live in tcbwd.cuh");
+  static_assert(MODE == 0 || MODE == 1 || MODE == 4 || MODE == 5, "row gradients live in tcbwd.cuh");
+  constexpr bool SQRT = MODE >= 4;
   extern __shared__ __align__(1024) unsigned char smem[];
   const int a_bytes = kTcM * kp * 2;
   const int b_bytes = BN * kp * 2 + BN * 4;
@@ -282,7 +305,13 @@ __global__ void __launch_bounds__(C::THREADS, 1)
       __syncwarp();
       if (lane == 0) mbar_arrive(bar_a);
     }
-    float acc[RT];                 // MODE 0: weighted sums
+    float cs = 1.f, cq = 0.f, c2 = 0.f;  // sqrt kernels: extent s, clamp on the scaled d^2, exponent per unit of r
+    if constexpr (SQRT) {
+      cs = tc_coord_scale(coord_absmax);
+      cq = clampq / cs / cs;
+      c2 = -kc * cs;
+    }
+    float acc[RT];                 // MODE 0, 4, 5: weighted sums
     float m[RT], srun[RT];         // MODE 1: running (m, s)
 #pragma unroll
     for (int r = 0; r < RT; ++r) {
@@ -302,12 +331,13 @@ __global__ void __launch_bounds__(C::THREADS, 1)
         for (int c0 = 0; c0 < CW; c0 += 32) {
           float v[32];
           tmem_ld32(lane_base + r * BN + half * CW + c0, v);
-          if constexpr (MODE == 0) {
+          if constexpr (MODE != 1) {
             if (self_mode) {
               // rows and columns are the SAME cloud (the K_xx / K_yy terms of an MMD): the exponent of the pair
               // (i, i) is -|X_i - X_i|^2/2 = 0 exactly, but the expansion X.X - |X|^2/2 - |X|^2/2 cancels three
               // O(|x/blur|^2) numbers in fp32 (5e-3 at blur = .05, D = 64 — BASELINE configs[2], where the diagonal
-              // IS the loss).  Warp-uniform test, taken on one column tile in N/128.
+              // IS the loss; for the sqrt kernels, r_ii = sqrt(fp32 noise) instead of sqrt(clamp)).  Warp-uniform
+              // test, taken on one column tile in N/128.
               const int64_t col0 = (int64_t)(t0 + k) * BN + half * CW + c0;
               const int64_t row_lo = (int64_t)(row_tile0 + r) * kTcM + quarter * 32;
               if (col0 < row_lo + 32 && row_lo < col0 + 32) {
@@ -317,14 +347,26 @@ __global__ void __launch_bounds__(C::THREADS, 1)
                   if (c == diag) v[c] = 0.f;
               }
             }
+            if constexpr (SQRT) {
+#pragma unroll
+              for (int c = 0; c < 32; ++c) {
+                // d^2 >= cq >= 0; r = d^2 rsqrt(d^2) is 0, not NaN, at d^2 = 0 (unclamped, or the diagonal)
+                const float d2 = fmaxf(-2.f * v[c], cq);
+                const float r = d2 * rsqrt_approx(fmaxf(d2, 1e-30f));
+                v[c] = (MODE == 4) ? ex2_approx(c2 * r) : r;
+              }
+            } else {
+#pragma unroll
+              for (int c = 0; c < 32; ++c) v[c] = ex2_approx(v[c]);
+            }
             const float4* w4 = reinterpret_cast<const float4*>(wts + half * CW + c0);
 #pragma unroll
             for (int c = 0; c < 32; c += 4) {
               const float4 w = w4[c / 4];
-              ts0 = fmaf(ex2_approx(v[c + 0]), w.x, ts0);
-              ts1 = fmaf(ex2_approx(v[c + 1]), w.y, ts1);
-              ts0 = fmaf(ex2_approx(v[c + 2]), w.z, ts0);
-              ts1 = fmaf(ex2_approx(v[c + 3]), w.w, ts1);
+              ts0 = fmaf(v[c + 0], w.x, ts0);
+              ts1 = fmaf(v[c + 1], w.y, ts1);
+              ts0 = fmaf(v[c + 2], w.z, ts0);
+              ts1 = fmaf(v[c + 3], w.w, ts1);
             }
           } else {
             float cs0 = 0.f, cs1 = 0.f;
@@ -355,7 +397,7 @@ __global__ void __launch_bounds__(C::THREADS, 1)
             ts1 += cs1;
           }
         }
-        if constexpr (MODE == 0) {
+        if constexpr (MODE != 1) {
           acc[r] += ts0 + ts1;
         } else {
           srun[r] += ts0 + ts1;
@@ -372,8 +414,8 @@ __global__ void __launch_bounds__(C::THREADS, 1)
     for (int r = 0; r < RT; ++r) {
       const int64_t row = (int64_t)(row_tile0 + r) * kTcM + quarter * 32 + lane;
       if (row < N) {
-        if constexpr (MODE == 0) {
-          part[((int64_t)split * NH + half) * N + row] = acc[r];
+        if constexpr (MODE != 1) {
+          part[((int64_t)split * NH + half) * N + row] = (MODE == 5) ? cs * acc[r] : acc[r];
         } else {
           reinterpret_cast<float2*>(part)[((int64_t)split * NH + half) * N + row] = make_float2(m[r], srun[r]);
         }

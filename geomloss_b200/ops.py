@@ -73,7 +73,7 @@ def _f32c(t, name):
     return t.contiguous()
 
 
-MAX_D_TC = 64  # softmin (p = 2) and gaussian kernel convolution, forward + row gradients: tensor-core path, 8 < D <= 64
+MAX_D_TC = 64  # softmin (p = 2) and kernel convolutions, forward + row gradients: tensor-core path, 8 < D <= 64
 
 
 def _check_clouds(x, y, max_d=None):
@@ -85,7 +85,8 @@ def _check_clouds(x, y, max_d=None):
     if x.shape[1] > max_d:
         raise NotImplementedError(f"D = {x.shape[1]} > {max_d}: not instantiated in this build (CUDA-core kernels "
                                   f"serve D <= {MAX_D}; the tensor-core kernels serve the p = 2 softmin and the "
-                                  f"gaussian kernel, forward and row gradients, up to D = {MAX_D_TC})")
+                                  f"gaussian / laplacian / energy kernel convolutions, forward and row gradients, "
+                                  f"up to D = {MAX_D_TC})")
     if x.device != y.device:
         raise ValueError("x and y must be on the same device")
 
@@ -243,7 +244,7 @@ def kind_id(kind):
 def kernel_conv_raw(kind, x, y, w, blur, *, center=None):
     """out_i = sum_j k(x_i, y_j) w_j, no autograd."""
     x, y, w, center = _f32c(x, "x"), _f32c(y, "y"), _f32c(w, "w"), _f32c(center, "center")
-    _check_clouds(x, y, MAX_D_TC if (kind_id(kind) & 0xFF) == 0 else MAX_D)
+    _check_clouds(x, y, MAX_D_TC)
     N, D = x.shape
     M = y.shape[0]
     if w.numel() != M:
@@ -264,7 +265,7 @@ def kernel_conv_raw(kind, x, y, w, blur, *, center=None):
 def kernel_conv_grad_rows(kind, x, y, w, blur, grad_out, *, center=None):
     x, y, w, center = _f32c(x, "x"), _f32c(y, "y"), _f32c(w, "w"), _f32c(center, "center")
     grad_out = _f32c(grad_out, "grad_out")
-    _check_clouds(x, y, MAX_D_TC if (kind_id(kind) & 0xFF) == 0 else MAX_D)
+    _check_clouds(x, y, MAX_D_TC)
     N, D = x.shape
     M = y.shape[0]
     dev = x.device

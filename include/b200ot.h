@@ -191,10 +191,12 @@ B200OT_API int b200ot_softmin_bwd_finalize(const float* part, int32_t n_part, co
 /* ---------------------------------------------------------------------------------------------
  * Kernel convolution  —  out_i = sum_j k(x_i, y_j) * w_j      (kernel_samples.py:128-137)
  * ------------------------------------------------------------------------------------------- */
-/* The gaussian kernel (forward and row gradients) additionally accepts 8 < D <= 64: that range runs on the tensor
- * cores (tcgen05, fp16x2 split operands, exponent accumulated in TMEM); laplacian / energy are limited to
- * D <= B200OT_MAX_D.  For D <= B200OT_MAX_D the library picks the faster of the two paths per operator and problem
- * size (csrc/b200ot_kernel_conv.cu: tc_routed); results agree to the tolerances of DESIGN.md section 4 either way. */
+/* Forward and row gradients additionally accept 8 < D <= 64 for every kind: that range runs on the tensor cores
+ * (tcgen05, fp16x2 split operands, -|x - y|^2 / 2 accumulated in TMEM; laplacian / energy take the square root in the
+ * epilogue, on coordinates scaled by the extent of the clouds, with or without B200OT_KERNEL_UNCLAMPED).  For
+ * D <= B200OT_MAX_D the library picks the faster of the two paths per operator and problem size for the gaussian
+ * (csrc/b200ot_kernel_conv.cu: tc_routed); laplacian / energy stay on the CUDA cores there.  Results agree to the
+ * tolerances of DESIGN.md section 4 either way. */
 B200OT_API int64_t b200ot_kernel_conv_scratch_bytes(int64_t N, int64_t M, int32_t D);
 
 B200OT_API int b200ot_kernel_conv_fwd(const float* x, const float* y, const float* w, const float* center, float* out,

@@ -101,6 +101,16 @@ if "tc" in which:
         check(f"tc_softmin_d{d}", sm, ref_softmin(1.0, x, y, h, 2), 1e-4)
         (gx,) = torch.autograd.grad(sm.sum(), xg)
         assert torch.isfinite(gx).all()
+        # laplacian / energy (MODE 4 / 5 of the forward and row-gradient kernels), cross and self (x is y)
+        for kind in ("laplacian", "energy"):
+            K = {"laplacian": (-(d2 / 4.0).clamp_min(1e-8).sqrt()).exp(), "energy": -d2.clamp_min(1e-8).sqrt()}[kind]
+            out = ops.kernel_conv(kind, xg, y.to(DEV), w.to(DEV), 2.0)
+            check(f"tc_conv_{kind}_d{d}", out, (K @ w.double()).float(), 1e-4)
+            (gx,) = torch.autograd.grad(out.sum(), xg)
+            assert torch.isfinite(gx).all()
+            out = ops.kernel_conv(kind, xg, xg.detach(), w[:700].to(DEV), 2.0)
+            (gx,) = torch.autograd.grad(out.sum(), xg)
+            assert torch.isfinite(out).all() and torch.isfinite(gx).all()
 if "grid" in which:
     for shape in ((1, 2, 32, 32), (1, 1, 16, 16, 16), (1, 1, 1024, 1024)):
         h = torch.randn(*shape, generator=g)
